@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on BASELINE.json's config, on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--skip-configs]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--skip-configs] [--dump-outputs DIR]
 
 metric  : XSimGCL yelp2018 train steps/sec (+ full-catalog rank items/sec as `rank`)
 workload: configs[2] of BASELINE.json -- XSimGCL, yelp2018 shape (31 668 x 38 048 x 1 237 259, synthetic power-law
@@ -19,8 +19,13 @@ Other configs of BASELINE.json ride along as sub-records of the same JSON line: 
 `config4` (SGL edge-drop, amazon-kindle shape, view graphs rebuilt on the device), `config5` (SimGCL, synthetic
 10 M x 2 M x 200 M, d = 128; single GPU at N = 1, bipartite-sharded at N > 1).
 --impl reference times the reference's own CPU path on the host cores: the UNMODIFIED reference unpacked from
-baseline/_ref/reference.zip (kind "reference") when that archive travelled, else the op-for-op port
+oracle/_ref/reference.zip (kind "reference") when build() made that archive, else the op-for-op port
 oracle/torch_port.py (kind "port"); rank 0 only; best of a thread-count sweep.
+--dump-outputs DIR (N = 1) writes what the last timed step left to its caller -- user_emb [U, d], item_emb [I, d] and
+the four losses, float32 -- as DIR/<name>.npy (17.8 MB).  The inputs are seeded: the same arguments give the same
+inputs on every run, so two builds can be compared output for output.  The step adds its gradient scatters with
+atomics, so two runs of one build agree closely but not bit for bit (two pairs of runs, --steps 20 --warmup 5 on a B200
+at 1000 W: tables within 5e-3 in relative Frobenius norm, losses within 1e-4 relative); compare with a tolerance.
 """
 import argparse
 import json
@@ -122,6 +127,23 @@ class ClockSampler:
         if not sm:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["no samples"]}
         return {"sm_mhz": float(np.median(sm)), "sm_max_mhz": float(max(mx)), "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: float32 / float64 array} as out_dir/<name>.npy; at most DUMP_LIMIT_BYTES in all."""
+    arrays = {k: np.ascontiguousarray(v) for k, v in arrays.items()}
+    for k, v in arrays.items():
+        if v.dtype not in (np.float32, np.float64):
+            raise ValueError(f"--dump-outputs: {k} is {v.dtype}, not float32 / float64")
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the limit of {DUMP_LIMIT_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v)
 
 
 def spmm_bytes(n, nnz, d):
@@ -291,7 +313,7 @@ def run_reference(args, rank, world):
     dt = cpu.run(steps, warm)
     val = steps / dt
     rdt, r_users, r_items = cpu.rank()
-    note = ("UNMODIFIED reference (baseline/_ref/reference.zip): its own XSimGCL.train() loop, sampler, losses, torch.optim.Adam"
+    note = ("UNMODIFIED reference (oracle/_ref/reference.zip): its own XSimGCL.train() loop, sampler, losses, torch.optim.Adam"
             if cpu.kind == "reference" else "op-for-op port of the reference's CPU path (oracle/torch_port.py) incl. Python sampler")
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": "steps/s", "n_gpus": args.gpus, "steps": steps, "warmup": warm,
@@ -562,6 +584,9 @@ def run_single(args, local_rank):
         resident_step(k)
     clocks.start()
     ms = time_steps(resident_step, args.steps, 0, torch)
+    outputs = None
+    if args.dump_outputs:  # the last timed step's results, taken before keep_load steps on
+        outputs = {"user_emb": eng.user_emb.cpu().numpy(), "item_emb": eng.item_emb.cpu().numpy(), "losses": eng.losses.cpu().numpy()}
     keep_load(resident_step, ms / args.steps, torch)  # nvidia-smi needs ~0.4 s of this same load to see it
     clk = clocks.stop()
     clk["window"] = "timed region + 0.4 s of the same graph-replay loop (keep_load)"
@@ -699,6 +724,8 @@ def run_single(args, local_rank):
                 line[name] = {"error": f"{type(e).__name__}: {e}"}
             line[name]["wall_s"] = time.perf_counter() - t0
             torch.cuda.empty_cache()
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     emit(line)
 
 
@@ -869,11 +896,14 @@ def main():
     ap.add_argument("--profile", action="store_true", help="eager steps only, for ncu (never a bench value)")
     ap.add_argument("--skip-configs", action="store_true", help="headline metric only (no config2/4/5 sub-records)")
     ap.add_argument("--skip-cpu", action="store_true", help="no cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's parameters and losses as DIR/<name>.npy")
     args = ap.parse_args()
-    claim_stdout()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl != "ours" or args.profile or world > 1):
+        ap.error("--dump-outputs covers the single-process timed path (--impl ours, one GPU, no --profile)")
+    claim_stdout()
     if args.impl == "reference":
         run_reference(args, rank, world)
         return

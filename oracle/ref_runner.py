@@ -1,6 +1,6 @@
 """TEST / BENCH INFRASTRUCTURE -- never imported by the product.
 
-Runs the UNMODIFIED reference (unpacked from baseline/_ref/reference.zip by oracle/refarchive.py) on the host CPUs
+Runs the UNMODIFIED reference (unpacked from oracle/_ref/reference.zip by oracle/refarchive.py) on the host CPUs
 for bench.py's reference arm: the reference's own XSimGCL class, its own train() loop, its own sampler, losses,
 encoder and torch.optim.Adam.  Harness-side shims only (SURVEY 8c; no edits to the reference):
   * cwd = a scratch directory (the reference writes ./log/),

@@ -1,19 +1,17 @@
 """TEST / BENCH INFRASTRUCTURE -- never imported by the product (selfrec_b200/).
 
-The unmodified reference cannot travel to the GPU box as a directory of sources in this repo, and it is pure Python
-without a setup.py, so `pip install --target baseline/_ref /root/reference` has nothing to install.  What travels
-instead is ONE git-ignored archive, baseline/_ref/reference.zip, made here (where /root/reference exists) by
-__graft_entry__.build(): the reference's .py / .yaml files plus the three datasets BASELINE.json's configs name
-(douban-book, yelp2018, amazon-kindle).  On the GPU box it is unpacked into a scratch directory by
+The unmodified reference is pure Python without a setup.py and its sources are not part of this repository.  Where a
+checkout of it is at hand, __graft_entry__.build() packs it once into the git-ignored archive oracle/_ref/reference.zip:
+the reference's .py / .yaml files plus the three datasets BASELINE.json's configs name (douban-book, yelp2018,
+amazon-kindle).  Where the archive exists it is unpacked into a scratch directory by
   * tests/test_gpu_reference_files.py  (the reference's own model files running on the drop-in modules),
   * bench.py --impl reference / the cpu_baseline leg (the reference's own CPU path, kind "reference"),
-  * the real-file full-size parity tests,
-all of which fall back (port / synthetic shape / skip) when the archive is absent."""
+all of which fall back (port / skip) when the archive is absent."""
 import os
 import zipfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-ARCHIVE = os.path.join(ROOT, "baseline", "_ref", "reference.zip")
+ARCHIVE = os.path.join(ROOT, "oracle", "_ref", "reference.zip")
 DATASETS = ("douban-book", "yelp2018", "amazon-kindle")
 
 

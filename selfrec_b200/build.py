@@ -41,7 +41,7 @@ def _digest():
     files = [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC))] + [os.path.join(INCLUDE, "selfrec_b200.h")]
     for f in files:
         with open(f, "rb") as fh:
-            h.update(f.encode())
+            h.update(os.path.relpath(f, ROOT).encode())  # not the absolute path: a moved tree keeps its build
             h.update(fh.read())
     h.update(" ".join(NVCC_FLAGS).encode())
     return h.hexdigest()

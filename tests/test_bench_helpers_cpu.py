@@ -68,3 +68,26 @@ def test_peaks_come_from_the_driver_file_when_present():
             assert pk["hbm_gbs"] == float(json.load(f)["hbm_gbs"]) and pk["source"].startswith("measured")
     else:
         assert pk["source"].startswith("fallback")
+
+
+def test_dump_outputs_writes_float_arrays_within_the_limit(tmp_path):
+    import numpy as np
+    import pytest
+    b = _bench()
+    arrays = {"emb": np.arange(12, dtype=np.float32).reshape(3, 4), "losses": np.array([0.5, 1.5], dtype=np.float64)}
+    b.dump_outputs(str(tmp_path / "out"), arrays)
+    for k, v in arrays.items():
+        got = np.load(tmp_path / "out" / f"{k}.npy")
+        assert got.dtype == v.dtype and np.array_equal(got, v)
+    with pytest.raises(ValueError):
+        b.dump_outputs(str(tmp_path / "int"), {"ids": np.arange(4, dtype=np.int32)})
+    with pytest.raises(ValueError):
+        b.dump_outputs(str(tmp_path / "big"), {"x": np.zeros(b.DUMP_LIMIT_BYTES // 4 + 1, dtype=np.float32)})
+    assert not (tmp_path / "int").exists() and not (tmp_path / "big").exists()
+
+
+def test_dump_outputs_is_refused_where_there_is_no_single_gpu_timed_path(tmp_path):
+    for extra, env in ((["--impl", "reference"], {}), (["--profile"], {}), ([], dict(RANK="1", WORLD_SIZE="2", LOCAL_RANK="1"))):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--dump-outputs", str(tmp_path)] + extra,
+                           capture_output=True, text=True, env=dict(os.environ, **env), timeout=120)
+        assert r.returncode == 2 and "--dump-outputs" in r.stderr and r.stdout == ""

@@ -1,7 +1,7 @@
 """The reference's OWN model files, unmodified, running on the drop-in modules on the GPU.
 
-Needs baseline/_ref/reference.zip (made by __graft_entry__.build() where /root/reference exists; it is the only
-form in which the reference travels to the GPU box -- oracle/refarchive.py) and is skipped without it.
+Needs oracle/_ref/reference.zip (made by __graft_entry__.build() where a checkout of the reference is at hand --
+oracle/refarchive.py) and is skipped without it: the reference's sources are not part of this repository.
 
   * install(fused_models=False): model/graph/{LightGCN,XSimGCL,SimGCL}.py are imported from the reference tree
     and trained for the three recorded batches of tests/golden/train_*.npz (same initial tables, same batches,
@@ -35,7 +35,7 @@ def ref_root(tmp_path_factory, built_lib):
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import refarchive
     if not refarchive.available():
-        pytest.skip("baseline/_ref/reference.zip is absent (built where /root/reference exists)")
+        pytest.skip("oracle/_ref/reference.zip is absent (build() makes it where a checkout of the reference is at hand)")
     return refarchive.unpack(str(tmp_path_factory.mktemp("reference")))
 
 
